@@ -6,12 +6,19 @@ sharded across N GPUs (one process per GPU, NCCL all-reduce inside the solver).
   python bench.py --gpus 1 --steps 3 --warmup 3
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
   python bench.py --impl reference ...      (CPU arm: the oracle port on host cores)
+  python bench.py ... --dump-outputs DIR    (also write the last timed step's results as DIR/<name>.npy)
 
 One "step" = one BundleAdjuster solve (cap of --lm-iters LM iterations, natural
 Ceres termination) from the same perturbed start; `value` = observations x LM
 iterations / device time with the problem resident in HBM; `e2e` = the same
 through the one-shot C-ABI call b200sfm_ba_solve with pinned HOST buffers
 (upload, structure build, solve, download inside the timed region).
+
+--dump-outputs writes, after the timed steps, what the last one computed: the
+refined quat / trans / points / intr_params and cost = [initial, final] (float64;
+under N GPUs each rank writes its own point shard as points_rank<r>.npy), or for
+config5 the estimated rotations [frames, 3, 3].  The inputs are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -50,6 +57,18 @@ WORKLOADS = {
     "tiny": (200, 20_000, 8.0, 2_500),
 }
 CPU_SAMPLE = "config2"   # bounded sample for the CPU baseline: 1/10 of the cameras and points
+DUMP_LIMIT_BYTES = 64 << 20   # --dump-outputs: the largest workload (config4) writes ~48.6 MB
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Write each array as out_dir/<name>.npy in float64; refuses more than DUMP_LIMIT_BYTES in all."""
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES} byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
 
 
 def peaks():
@@ -415,6 +434,12 @@ def run_b200(args):
     for r in (roof_mv, roof_li):
         r["frac"] = r["achieved"] / peak if r["achieved"] else None
     final_cost, init_cost = stats[-1]["final_cost"], stats[-1]["initial_cost"]
+    if args.dump_outputs:
+        intr, quat, trans, points = prob.get_state()
+        out = {"points" if world == 1 else f"points_rank{rank}": points}
+        if rank == 0:   # cameras and costs are replicated on every rank
+            out.update(quat=quat, trans=trans, intr_params=intr, cost=np.array([init_cost, final_cost]))
+        dump_outputs(args.dump_outputs, out)
     prob.free()
 
     # ---- end-to-end leg: one-shot C-ABI call with pinned host buffers ----------------
@@ -520,15 +545,23 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true", help="skip the config-2 GPU-vs-CPU-port parity record")
     ap.add_argument("--design", type=int, default=0, help="BA data layout: 0 auto (v2), 1 = v1 (W blocks + atomics), 2 = v2")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float64, <= 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA path's results; the CPU arm (--impl reference) has none")
     if args.workload == "config5":
         # BASELINE.json config 5 (100 k-frame view graph): rotation averaging, the secondary metric of SURVEY.md 8(d)
         # (edges/s per L1 / IRLS iteration).  Single GPU; the line is printed by bench_secondary.py in the same JSON style.
         if int(os.environ.get("RANK", "0")) != 0:
             return   # one GPU: under torchrun only rank 0 measures
         import bench_secondary as B2
-        B2.bench_ra(argparse.Namespace(frames=100_000, neighbours=100, steps=max(1, min(args.steps, 3)), warmup=min(args.warmup, 1),
-                                       pcg_tol=1e-6))
+        R = B2.bench_ra(argparse.Namespace(frames=100_000, neighbours=100, steps=args.steps, warmup=min(args.warmup, 1),
+                                           pcg_tol=1e-6))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"rotations": R})
         return
     if args.impl == "reference":
         run_reference(args)

@@ -93,6 +93,7 @@ def bench_ra(args):
             "median_pair_error_deg": float(np.median(err)), "p99_pair_error_deg": float(np.percentile(err, 99)),
             "pcg_rel_tolerance": args.pcg_tol, "kernel_launches": st["kernel_launches"]}
     print(json.dumps(line))
+    return R
 
 
 if __name__ == "__main__":

@@ -1,10 +1,14 @@
 """Host logic of bench.py that does not need a GPU: the clock sampler's handling of nvidia-smi rows (the timed region of
 the default run is ~150 ms, shorter than nvidia-smi's start-up, so the rows carry timestamps and are filtered to it) and
-its graceful behaviour without NVML / nvidia-smi."""
+its graceful behaviour without NVML / nvidia-smi; the --dump-outputs writer and the argument checks."""
 import datetime
 import importlib.util
 import os
+import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -39,3 +43,21 @@ def test_sampler_without_a_gpu_reports_no_samples_instead_of_failing():
     out = s.stop()
     assert out["samples"] == 0 or out["sm_mhz"] is not None
     assert set(out) >= {"sm_mhz", "sm_max_mhz", "reasons", "samples"}
+
+
+def test_dump_outputs_writes_float64_and_refuses_more_than_the_limit(tmp_path):
+    B = _bench()
+    B.dump_outputs(str(tmp_path / "out"), {"points": np.arange(6, dtype=np.float32).reshape(2, 3), "cost": [2.0, 1.0]})
+    pts, cost = np.load(tmp_path / "out" / "points.npy"), np.load(tmp_path / "out" / "cost.npy")
+    assert pts.dtype == np.float64 and pts.shape == (2, 3) and pts[1, 2] == 5.0
+    assert cost.dtype == np.float64 and cost.tolist() == [2.0, 1.0]
+    with pytest.raises(SystemExit):
+        B.dump_outputs(str(tmp_path / "big"), {"points": np.zeros(B.DUMP_LIMIT_BYTES // 8 + 1)})
+    assert not (tmp_path / "big").exists()
+
+
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "x"]])
+def test_bench_rejects_arguments_it_cannot_honour(argv, tmp_path):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + argv, cwd=tmp_path, capture_output=True, text=True)
+    assert r.returncode == 2 and "error" in r.stderr, r.stderr
+    assert not (tmp_path / "x").exists()
